@@ -4,6 +4,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --steps K --warmup W    # the reference's algorithm on host cores
+    python bench.py ... --dump-outputs DIR                   # also save the last timed step's records as DIR/*.npy
 
 One "step" = one full pass of the hot path (encoder, 9 constrained decode steps, hypothesis records, the
 single gather of the records to rank 0) over the 1 000-query batch.  With N GPUs the SAME 1 000 queries are
@@ -220,6 +221,8 @@ def run_ours(args):
     full = merge_gathered(gathered, layout) if (world > 1 and rank == 0) else (rec.host() if world == 1 else None)
     errs = rec.host()["errors"] if Q else np.zeros(4, dtype=np.int32)
     assert not errs.any(), f"generate raised error flags {errs.tolist()} (include/sealdec.h)"
+    if args.dump_outputs and full is not None:
+        dump_outputs(full, args.dump_outputs)
 
     # ---- end to end through the public host-array API: H2D of the inputs, decode, the gather, D2H of the records ----
     e2e_steps = max(1, min(args.steps, 3))
@@ -322,6 +325,35 @@ def run_ours(args):
     if weak:
         out["weak"] = weak
     print(json.dumps(out))
+
+
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(rec, out_dir, limit=DUMP_LIMIT):
+    """Writes the hypothesis records of the last timed step (what the caller of the timed path receives) as
+    out_dir/<name>.npy: SA bounds as float64, everything else as float32 (token ids, lengths and flags are exact there).
+    A slot without a hypothesis has score -inf in the records; the dump marks such slots 0 in present.npy and stores
+    score 0 there, so every written value is finite.
+    If the records exceed `limit` bytes, a fixed seeded sample of queries is written, their indices in query_index.npy."""
+    rec = dict(rec)
+    present = ~np.isneginf(rec["scores"])                      # a NaN stays in the dump: it would be a fault
+    rec["present"] = present.astype(np.uint8)
+    rec["scores"] = np.where(present, rec["scores"], np.float32(0))
+    per_dtype = {k: (np.float64 if v.dtype in (np.uint64, np.int64) else np.float32) for k, v in rec.items()}
+    Q = rec["scores"].shape[0]
+    row_bytes = sum(np.dtype(per_dtype[k]).itemsize * rec[k][0].size for k in rec if k != "errors") if Q else 0
+    rows = None
+    if Q and Q * row_bytes > limit - 4096:                     # 4 KB left for the .npy headers
+        n = (limit - 4096) // (row_bytes + 8)
+        rows = np.sort(np.random.default_rng(0).choice(Q, size=n, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in rec.items():
+        if rows is not None and k != "errors":
+            v = v[rows]
+        np.save(os.path.join(out_dir, k + ".npy"), v.astype(per_dtype[k]))
+    if rows is not None:
+        np.save(os.path.join(out_dir, "query_index.npy"), rows.astype(np.float64))
 
 
 def rank_kernel_report(index, full, dev, hbm, phases, args):
@@ -547,7 +579,11 @@ def main():
     ap.add_argument("--no-big-index", action="store_true")
     ap.add_argument("--no-gpu-eager-baseline", action="store_true")
     ap.add_argument("--big-index-tokens", type=int, default=200_000_000)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the hypothesis records of the last timed step as DIR/<name>.npy (at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -204,19 +204,29 @@ def _host_build(text):
     return fm
 
 
-def test_sdsl_format_writer_round_trip_and_reference_bytes(tmp_path):
-    """FMIndex.save writes the reference's own .fmi format: (1) our loader reads it back to identical sections;
-    (2) where the compiled reference is available the file is byte-identical to the reference's FMIndex::save of the
-    same text (both select_support_mcl construction paths, contiguous and sparse alphabets, long select blocks)."""
-    import numpy as np
-    from oracle.fm_oracle import RefFM, ref_available
-    from seal_b200.cpp_modules.fm_index import load_FMIndex
+def sdsl_writer_texts():
+    """The texts of the .fmi writer test (both select_support_mcl construction paths, contiguous and sparse alphabets,
+    long select blocks); tests/golden/make_fmi_golden.py saves each with the reference's FMIndex::save."""
     from seal_b200.synthetic import make_corpus, corpus_symbols
     rng = np.random.default_rng(1)
-    texts = {"toy": [12, 13, 12, 14, 13, 12], "one": [5], "contiguous": rng.integers(1, 6, size=300),
-             "rand5k": rng.integers(10, 300, size=5000), "wide": rng.integers(10, 50000, size=7000),
-             "phrase 40k": corpus_symbols(make_corpus(n_docs=400, doc_len=100, n_phrases=600, seed=4)),   # tree > 100 000 bits
-             "run": np.full(9000, 11), "sparse": np.array([2 ** 15] + [1] * 20000, dtype=np.uint64)}
+    return {"toy": [12, 13, 12, 14, 13, 12], "one": [5], "contiguous": rng.integers(1, 6, size=300),
+            "rand5k": rng.integers(10, 300, size=5000), "wide": rng.integers(10, 50000, size=7000),
+            "phrase 40k": corpus_symbols(make_corpus(n_docs=400, doc_len=100, n_phrases=600, seed=4)),   # tree > 100 000 bits
+            "run": np.full(9000, 11), "sparse": np.array([2 ** 15] + [1] * 20000, dtype=np.uint64)}
+
+
+def test_sdsl_format_writer_round_trip_and_reference_bytes(tmp_path):
+    """FMIndex.save writes the reference's own .fmi format: (1) our loader reads it back to identical sections;
+    (2) the file is byte-identical to the reference's FMIndex::save of the same text, whose length and SHA-256 are
+    stored in tests/golden/fmi_golden.json."""
+    import hashlib
+    import json
+    import numpy as np
+    from seal_b200.cpp_modules.fm_index import load_FMIndex
+    with open(os.path.join(HERE, "golden", "fmi_golden.json")) as f:
+        ref_files = json.load(f)["files"]
+    texts = sdsl_writer_texts()
+    assert sorted(texts) == sorted(ref_files)
     for name, text in texts.items():
         fm = _host_build(text)
         ours = str(tmp_path / "ours.fmi")
@@ -224,10 +234,8 @@ def test_sdsl_format_writer_round_trip_and_reference_bytes(tmp_path):
         back = load_FMIndex(ours)
         for w in range(5):
             assert np.array_equal(fm.section(w), back.section(w)), (name, w)
-        if ref_available():
-            ref = str(tmp_path / "ref.fmi")
-            RefFM(np.asarray(text, dtype=np.uint64)).save(ref)
-            assert open(ours, "rb").read() == open(ref, "rb").read(), name
+        data = open(ours, "rb").read()
+        assert {"bytes": len(data), "sha256": hashlib.sha256(data).hexdigest()} == ref_files[name], name
         nat = str(tmp_path / "ours.native")
         fm.save(nat, native=True)
         assert np.array_equal(load_FMIndex(nat).section(0), fm.section(0))
