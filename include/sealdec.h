@@ -176,6 +176,11 @@ int sealdec_debug_step_logits(sealbart_t* model, const int64_t* input_ids, const
  * device time per call (CUDA events, includes the activation split). */
 int sealdec_debug_gemm(int mode, int64_t M, int32_t N, int32_t K, const float* A, const float* W,
                        const float* bias, float* C, int32_t gelu, int32_t iters, double* avg_us);
+/* The same GEMM with the output written as the fp16 split (h1, h2) that the next 3xFP16 GEMM consumes (modes 3 and 5):
+ * halves_sum float32 [M][N] host receives h1 + h2; *overflow (may be NULL) = 1 if an output left the fp16 range
+ * (|x| > 65504, saturated), else 0. */
+int sealdec_debug_gemm_split(int mode, int64_t M, int32_t N, int32_t K, const float* A, const float* W,
+                             const float* bias, int32_t gelu, float* halves_sum, int32_t* overflow);
 /* in-kernel timeline of CTA 0 of the mode-3/4 GEMM kernel (development aid): out20 (may be NULL) receives
  * the stamps of the last traced launch -- SM cycles at 0 entry, 1 prologue done, 2 first operands landed,
  * 3 last MMA issued, 4 last chunk complete, 5 tile stored, 6 exit; 7/8 globaltimer ns at entry / exit --

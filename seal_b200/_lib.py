@@ -111,6 +111,7 @@ _DEC_SIGS = {
     "sealdec_debug_step_logits": (i32, [vp, vp, vp, C.c_int64, C.c_int64, C.c_int32, vp, C.c_int64, vp]),
     "sealdec_debug_gemm": (i32, [i32, C.c_int64, C.c_int32, C.c_int32, vp, vp, vp, vp, C.c_int32, C.c_int32,
                                  C.POINTER(C.c_double)]),
+    "sealdec_debug_gemm_split": (i32, [i32, C.c_int64, C.c_int32, C.c_int32, vp, vp, vp, C.c_int32, vp, vp]),
     "sealdec_debug_gemm_trace": (i32, [i32, C.POINTER(C.c_int64)]),
     "sealev_first_stage": (i32, [C.c_int64, vp, vp, vp, vp, C.c_int64, vp, vp, vp, i32, i32, C.c_double, C.c_double, C.c_int64, vp, vp]),
     "sealev_score_docs": (i32, [C.c_int64, vp, vp, vp, vp, C.c_int64, C.c_int64, vp, vp, vp, C.c_int64, i32, i32, i32, i32,

@@ -185,16 +185,17 @@ EncodeTiledFn encode_tiled() {
     }
     return fn;
 }
-// row-major [rows][K] fp32 (or fp16), box = 128 bytes of K x box_rows, 128B swizzle, zero fill out of bounds
+// row-major [rows][K] fp32 (or fp16), box = row_bytes (128, 64 or 32) of K x box_rows, swizzled at the box's row width,
+// zero fill out of bounds
 void make_map(CUtensorMap* map, const void* ptr, uint64_t rows, uint64_t K, uint64_t ld, uint32_t box_rows, bool half = false,
               int row_bytes = 128) {
     cuuint64_t dims[2] = {K, rows};
     cuuint64_t strides[1] = {ld * (half ? 2 : 4)};
     cuuint32_t box[2] = {(cuuint32_t)(row_bytes / (half ? 2 : 4)), box_rows};
     cuuint32_t estr[2] = {1, 1};
+    const CUtensorMapSwizzle sw = row_bytes == 128 ? CU_TENSOR_MAP_SWIZZLE_128B : row_bytes == 64 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_32B;
     CUresult r = encode_tiled()(map, half ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, const_cast<void*>(ptr), dims, strides, box, estr,
-                                CU_TENSOR_MAP_INTERLEAVE_NONE, row_bytes == 128 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B,
-                                CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                                CU_TENSOR_MAP_INTERLEAVE_NONE, sw, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                                 CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (r != CUDA_SUCCESS) throw ApiError(SEALFM_ECUDA, "cuTensorMapEncodeTiled failed (" + std::to_string((int)r) + ")");
 }
@@ -308,10 +309,19 @@ void gemm_impl(Ctx& cx, int64_t M, int N, int K, const Act& A, int lda, Lin& l, 
             }
             float* part = nullptr;
             if (tail_s > 1) { m->splitk.ensure((size_t)(pair_tiles - full_items) * tail_s * 65536 * 4); part = m->splitk.as<float>(); }
+            // the epilogue stores boxes of 16 columns x 32 rows (umma_gemm_2cta.cuh); maps are passed by value, so a
+            // captured graph replays them as long as the buffers keep their addresses (g_ws_epoch)
+            const bool split_out = C.h1 != nullptr;
+            if (split_out == (C.x != nullptr) || (split_out && !C.h2)) throw ApiError(SEALFM_EINVAL, "internal: the CTA-pair GEMM writes either fp32 or fp16 halves");
+            CUtensorMap mo1, mo2, mpart;
+            if (split_out) { make_map(&mo1, C.h1, M, N, ldc, 32, true, 32); make_map(&mo2, C.h2, M, N, ldc, 32, true, 32); }
+            else { make_map(&mo1, C.x, M, N, ldc, 32, false, 64); mo2 = mo1; }
+            if (part) make_map(&mpart, part, (uint64_t)(pair_tiles - full_items) * tail_s * 256, 256, 256, 32, false, 64);
+            else mpart = mo1;
             auto launchp = [&](auto kern) {
                 CUDA_CHECK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, U2_SMEM));
-                launch_k(kern, 2 * pairs, UTHREADS2, U2_SMEM, cx.s, ma1, ma2, l.map2_hi, l.map2_lo, (int)M, N, K, l.b, l.w_unscale, C.x, C.h1, C.h2, ldc, n_fastest, ovf,
-                           full_items, tail_s, part);
+                launch_k(kern, 2 * pairs, UTHREADS2, U2_SMEM, cx.s, ma1, ma2, l.map2_hi, l.map2_lo, mo1, mo2, mpart, (int)M, N, K, l.b, l.w_unscale,
+                         (int)split_out, n_fastest, ovf, full_items, tail_s);
             };
             if (gelu) launchp(umma_gemm_f16x3_2cta_kernel<true>); else launchp(umma_gemm_f16x3_2cta_kernel<false>);
             CUDA_CHECK(cudaGetLastError()); m->launches++;
@@ -1296,18 +1306,24 @@ int sealdec_teacher_forced(sealbart_t* m, const int64_t* ids, const int64_t* mas
     });
 }
 
-int sealdec_debug_gemm(int mode, int64_t M, int32_t N, int32_t K, const float* A, const float* W, const float* bias, float* C,
-                       int32_t gelu, int32_t iters, double* avg_us) {
+}  // extern "C"
+
+namespace {
+// sealdec_debug_gemm / sealdec_debug_gemm_split: C is written as fp32 (C != nullptr) or as the fp16 halves the next GEMM
+// consumes, returned as their sum h1 + h2 in `halves_sum` with the producer's overflow flag in `overflow`
+int debug_gemm(int mode, int64_t M, int32_t N, int32_t K, const float* A, const float* W, const float* bias, float* C,
+               int32_t gelu, int32_t iters, double* avg_us, float* halves_sum, int32_t* overflow) {
     return guarded([&] {
-        if (!A || !W || !C || M <= 0 || N <= 0 || K <= 0) throw ApiError(SEALFM_EINVAL, "bad argument");
+        if (!A || !W || (!C && !halves_sum) || M <= 0 || N <= 0 || K <= 0) throw ApiError(SEALFM_EINVAL, "bad argument");
         int count = 0;
         if (cudaGetDeviceCount(&count) != cudaSuccess || count == 0) { cudaGetLastError(); throw ApiError(SEALFM_ENODEVICE, "no CUDA device available"); }
         if (mode != 2 && mode != 3 && mode != 5) throw ApiError(SEALFM_EINVAL, "gemm_mode must be 2, 3 or 5");
+        if (halves_sum && mode == 2) throw ApiError(SEALFM_EINVAL, "the fp16 split output exists in gemm_mode 3 and 5 only");
         sealbart fake; fake.cfg.gemm_mode = mode;
         CUDA_CHECK(cudaGetDevice(&fake.device));
         Buf dA, dW, dB, dC, whi, wlo;
         struct Rel { std::vector<Buf*> v; sealbart* f; ~Rel() { for (auto b : v) b->release(); f->a_hi.release(); f->a_lo.release(); f->err.release(); f->splitk.release(); } } rel{{&dA, &dW, &dB, &dC, &whi, &wlo}, &fake};
-        const int ldc = (N + 3) / 4 * 4;
+        const int ldc = halves_sum ? (N + 7) / 8 * 8 : (N + 3) / 4 * 4;        // 16-byte rows
         dA.ensure((size_t)M * K * 4); dW.ensure((size_t)N * K * 4); dB.ensure((size_t)N * 4); dC.ensure((size_t)M * ldc * 4);
         CUDA_CHECK(cudaMemcpy(dA.p, A, (size_t)M * K * 4, cudaMemcpyHostToDevice));
         CUDA_CHECK(cudaMemcpy(dW.p, W, (size_t)N * K * 4, cudaMemcpyHostToDevice));
@@ -1330,20 +1346,45 @@ int sealdec_debug_gemm(int mode, int64_t M, int32_t N, int32_t K, const float* A
             CUDA_CHECK(cudaGetLastError());
         }
         Ctx cx{&fake, nullptr};
-        gemm(cx, M, N, K, Act{dA.as<float>()}, K, l, Act{dC.as<float>()}, ldc, gelu != 0);
+        Act out;
+        if (halves_sum) { out.h1 = dC.as<__half>(); out.h2 = dC.as<__half>() + (size_t)M * ldc; }
+        else out.x = dC.as<float>();
+        gemm(cx, M, N, K, Act{dA.as<float>()}, K, l, out, ldc, gelu != 0);
         CUDA_CHECK(cudaDeviceSynchronize());
         if (iters > 0 && avg_us) {
             cudaEvent_t e0, e1; CUDA_CHECK(cudaEventCreate(&e0)); CUDA_CHECK(cudaEventCreate(&e1));
             CUDA_CHECK(cudaEventRecord(e0, nullptr));
-            for (int i = 0; i < iters; ++i) gemm(cx, M, N, K, Act{dA.as<float>()}, K, l, Act{dC.as<float>()}, ldc, gelu != 0);
+            for (int i = 0; i < iters; ++i) gemm(cx, M, N, K, Act{dA.as<float>()}, K, l, out, ldc, gelu != 0);
             CUDA_CHECK(cudaEventRecord(e1, nullptr));
             CUDA_CHECK(cudaEventSynchronize(e1));
             float ms = 0; CUDA_CHECK(cudaEventElapsedTime(&ms, e0, e1));
             *avg_us = (double)ms * 1e3 / iters;
             cudaEventDestroy(e0); cudaEventDestroy(e1);
         }
-        CUDA_CHECK(cudaMemcpy2D(C, (size_t)N * 4, dC.p, (size_t)ldc * 4, (size_t)N * 4, M, cudaMemcpyDeviceToHost));
+        if (halves_sum) {
+            std::vector<__half> h((size_t)2 * M * ldc);
+            CUDA_CHECK(cudaMemcpy(h.data(), dC.p, h.size() * 2, cudaMemcpyDeviceToHost));
+            for (int64_t r = 0; r < M; ++r)
+                for (int n = 0; n < N; ++n)
+                    halves_sum[r * N + n] = __half2float(h[r * ldc + n]) + __half2float(h[(size_t)M * ldc + r * ldc + n]);
+            if (overflow) CUDA_CHECK(cudaMemcpy(overflow, fake.ovf, 4, cudaMemcpyDeviceToHost));
+        } else {
+            CUDA_CHECK(cudaMemcpy2D(C, (size_t)N * 4, dC.p, (size_t)ldc * 4, (size_t)N * 4, M, cudaMemcpyDeviceToHost));
+        }
     });
+}
+}  // namespace
+
+extern "C" {
+
+int sealdec_debug_gemm(int mode, int64_t M, int32_t N, int32_t K, const float* A, const float* W, const float* bias, float* C,
+                       int32_t gelu, int32_t iters, double* avg_us) {
+    return debug_gemm(mode, M, N, K, A, W, bias, C, gelu, iters, avg_us, nullptr, nullptr);
+}
+
+int sealdec_debug_gemm_split(int mode, int64_t M, int32_t N, int32_t K, const float* A, const float* W, const float* bias,
+                             int32_t gelu, float* halves_sum, int32_t* overflow) {
+    return debug_gemm(mode, M, N, K, A, W, bias, nullptr, gelu, 0, nullptr, halves_sum, overflow);
 }
 
 int sealdec_apply_index_mask_d(const sealfm_t* fm, sealfm_stream_t stream, const sealdec_processor_cfg_t* cfg,

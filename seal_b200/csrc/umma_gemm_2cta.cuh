@@ -14,8 +14,15 @@
 //   empty[s]  one per CTA (count 1): the leader's MMA thread commits with .multicast::cluster to both.
 //   tfull[b]  one per CTA (count 1): multicast commit when a K chunk's partial sums are complete.
 //   tempty[b] leader's barrier only; count 2 x 16 epilogue warps; the peer's warps arrive remotely.
-// Each CTA's TMEM holds the accumulator rows of its own 128 rows (two 256-column buffers), so the epilogue is
-// the one-CTA kernel's.  Pair p walks pair-tiles p, p + #pairs, ...; a pair-tile = 256 rows x 256 columns.
+// Each CTA's TMEM holds the accumulator rows of its own 128 rows (two 256-column buffers).  Pair p walks
+// pair-tiles p, p + #pairs, ...; a pair-tile = 256 rows x 256 columns.
+//
+// Output: the MMA warp can run only two chunks (half a K = 1024 tile) ahead of the epilogue, so every cycle an
+// epilogue warp spends on a tile's output after its last chunk is a cycle the tensor pipe may wait.  Each
+// epilogue warp therefore finishes 16 columns of its 32 x 64 block at a time into a 2 KB shared-memory slot laid
+// out as a TMA box (lane = row) and hands the slot to one cp.async.bulk.tensor store; it waits for that store
+// to have read the slot only before refilling it.  The tensor maps clip at M and N, so ragged edges need no
+// code, and the raw partial sums of a K-sliced tail tile go out the same way through a map over `part`.
 #pragma once
 #include "umma_gemm.cuh"
 
@@ -25,7 +32,8 @@ constexpr int U2_STAGES = 3;
 constexpr int U2_AB = UM * 128;                       // one A tile (h1 or h2): 128 rows x 128 B
 constexpr int U2_WB = 128 * 128;                      // this CTA's half of the W tile: 128 rows x 128 B
 constexpr int U2_STAGE = 2 * U2_AB + 2 * U2_WB;       // 64 KB
-constexpr int U2_SMEM = U2_STAGES * U2_STAGE + 1024 /*alignment*/ + 256 /*barriers*/ + 16 * 2048 /*epilogue transpose*/;
+constexpr int U2_SLOT = 2048;                         // per epilogue warp: 32 rows x 16 fp32, or 32 x 16 h1 + 32 x 16 h2
+constexpr int U2_SMEM = U2_STAGES * U2_STAGE + 1024 /*alignment*/ + UEPI_WARPS * U2_SLOT + 256 /*barriers*/;
 
 __device__ __forceinline__ uint32_t cluster_ctarank() { uint32_t r; asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r)); return r; }
 __device__ __forceinline__ void cluster_sync_all() {
@@ -66,22 +74,42 @@ __device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t (&r)[16]) {
     asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
 }
 
+__device__ __forceinline__ void st_shared_v4(uint32_t addr, uint32_t a, uint32_t b, uint32_t c, uint32_t d) {
+    asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(addr), "r"(a), "r"(b), "r"(c), "r"(d) : "memory");
+}
+// shared -> global tensor store of one box at (c0 = column, c1 = row); elements outside the map are not written
+__device__ __forceinline__ void tma_store_2d(const CUtensorMap* map, uint32_t src, int c0, int c1) {
+    asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%2, %3}], [%1];"
+                 ::"l"(reinterpret_cast<uint64_t>(map)), "r"(src), "r"(c0), "r"(c1) : "memory");
+}
+__device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
+__device__ __forceinline__ void bulk_wait_read_all() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
+__device__ __forceinline__ void bulk_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
+// generic-proxy writes to shared memory become visible to the bulk-copy (async) proxy
+__device__ __forceinline__ void fence_proxy_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
+__device__ __forceinline__ uint32_t pack_half2(__half lo, __half hi) {
+    return (uint32_t)__half_as_ushort(lo) | ((uint32_t)__half_as_ushort(hi) << 16);
+}
+
 template <bool GELU>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(UTHREADS2, 1)
 umma_gemm_f16x3_2cta_kernel(const __grid_constant__ CUtensorMap tmA_hi, const __grid_constant__ CUtensorMap tmA_lo,
                             const __grid_constant__ CUtensorMap tmW_hi, const __grid_constant__ CUtensorMap tmW_lo,
-                            int M, int N, int K, const float* __restrict__ bias, float w_unscale, float* __restrict__ C,
-                            __half* __restrict__ C_h1, __half* __restrict__ C_h2, int ldc, int n_fastest,
-                            int* __restrict__ overflow, int full_items, int tail_s, float* __restrict__ part) {
+                            // output boxes of 16 columns x 32 rows: fp32 C (SWIZZLE_64B), or with split_out the fp16
+                            // halves h1 / h2 (SWIZZLE_32B); tmPart = the fp32 K-slice partial sums of the tail tiles
+                            const __grid_constant__ CUtensorMap tmOut, const __grid_constant__ CUtensorMap tmOut2,
+                            const __grid_constant__ CUtensorMap tmPart,
+                            int M, int N, int K, const float* __restrict__ bias, float w_unscale, int split_out, int n_fastest,
+                            int* __restrict__ overflow, int full_items, int tail_s) {
     constexpr int BN = 256, KE = 64, NST = U2_STAGES;
     constexpr int kChunkBlocks = UKC16;
     extern __shared__ uint8_t smem_raw[];
     const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
-    const uint32_t bars = base + NST * U2_STAGE;
+    const uint32_t slots = base + NST * U2_STAGE;               // 1024-aligned: the swizzle patterns repeat within a slot
+    const uint32_t bars = slots + UEPI_WARPS * U2_SLOT;
     const uint32_t full0 = bars, empty0 = bars + 8 * NST;
     const uint32_t tfull0 = bars + 16 * NST, tempty0 = tfull0 + 16;
     const uint32_t slot = tempty0 + 16;
-    float* stage_base = reinterpret_cast<float*>(smem_raw + (base - smem_u32(smem_raw)) + NST * U2_STAGE + 256);
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const uint32_t rank = cluster_ctarank();
     const int pair = blockIdx.x >> 1, n_pairs = gridDim.x >> 1;
@@ -93,7 +121,7 @@ umma_gemm_f16x3_2cta_kernel(const __grid_constant__ CUtensorMap tmA_hi, const __
     // Work list: items [0, full_items) are whole pair-tiles (all of K); the pair-tiles that would form a
     // mostly idle last wave are cut into tail_s K-slices each, so that wave costs 1/tail_s of a tile time:
     // item full_items + j = slice j % tail_s of pair-tile full_items + j / tail_s, raw partial sums stored to
-    // part[(tile - full_items) * tail_s + slice][256][256] (umma_tail_finish_kernel adds the slices in order).
+    // rows [j * 256, j * 256 + 256) of tmPart (umma_tail_finish_kernel adds the slices in order).
     const int total_items = full_items + (total - full_items) * tail_s;
     struct Item { int tile, kb0, nkb, slot; };
     auto decode = [&](int item) {
@@ -180,6 +208,7 @@ umma_gemm_f16x3_2cta_kernel(const __grid_constant__ CUtensorMap tmA_hi, const __
         const int q = warp & 3;
         const int cg = (warp - 4) >> 2;
         const uint32_t lead_tempty0 = map_to_cta(tempty0, 0);
+        const uint32_t stg = slots + (uint32_t)(warp - 4) * U2_SLOT;
         uint32_t ch = 0;
         for (int item = pair; item < total_items; item += n_pairs) {
             const int num_chunks = ((item < full_items ? num_k : num_k / tail_s) + kChunkBlocks - 1) / kChunkBlocks;
@@ -203,67 +232,70 @@ umma_gemm_f16x3_2cta_kernel(const __grid_constant__ CUtensorMap tmA_hi, const __
             }
             const Item w = decode(item);                      // (kept out of the chunk loop: register pressure)
             const int pm = n_fastest ? w.tile / n_tiles : w.tile % pm_tiles, n_tile = n_fastest ? w.tile % n_tiles : w.tile / pm_tiles;
-            const int m_tile = 2 * pm + (int)rank;
-            const int row0 = m_tile * UM + q * 32;
-            const int nb = n_tile * BN + cg * 64;
-            float* stg = stage_base + (warp - 4) * 512;
-            if (w.slot >= 0) {
-                // K-slice of a tail tile: raw sums, lane = row, 64 consecutive floats per lane (L2-resident scratch)
-                float* dst = part + ((int64_t)w.slot * 256 + rank * 128 + q * 32 + lane) * 256 + cg * 64;
+            const bool raw = w.slot >= 0;                     // K-slice of a tail tile: unscaled partial sums
+            // this warp's 32 x 64 block: rows [row0, row0 + 32), columns [col0, col0 + 64) of C, or of the tail slice
+            // (the rank is read again here so that nothing derived from it stays live across the chunk loop)
+            const int rk = (int)cluster_ctarank();
+            const int row0 = raw ? w.slot * 256 + rk * 128 + q * 32 : (2 * pm + rk) * UM + q * 32;
+            const int col0 = raw ? cg * 64 : n_tile * BN + cg * 64;
+            if (!raw && (row0 >= M || col0 >= N)) continue;
+            // bias of the 64 columns, two per lane; column j is broadcast from lane j % 32 when it is needed
+            float b_lo = 0.f, b_hi = 0.f;
+            if (bias && !raw) {
+                if (col0 + lane < N) b_lo = bias[col0 + lane];
+                if (col0 + 32 + lane < N) b_hi = bias[col0 + 32 + lane];
+            }
+            int ov = 0;
 #pragma unroll
-                for (int j = 0; j < 64; j += 4) *reinterpret_cast<float4*>(dst + j) = make_float4(acc[j], acc[j + 1], acc[j + 2], acc[j + 3]);
-            } else if (row0 < M && nb < N) {
+            for (int pass = 0; pass < 4; ++pass) {            // 16 columns = one box per pass
+                const int col = col0 + pass * 16;
+                if (!raw && col >= N) break;
+                float* v = acc + pass * 16;                   // finished in place
+                if (!raw) {
 #pragma unroll
-                for (int pass = 0; pass < 4; ++pass) {
-#pragma unroll
-                    for (int j4 = 0; j4 < 4; ++j4) {
-                        float v[4];
-#pragma unroll
-                        for (int u = 0; u < 4; ++u) {
-                            const int n = nb + pass * 16 + j4 * 4 + u;
-                            const float x = acc[pass * 16 + j4 * 4 + u] * w_unscale + ((bias && n < N) ? bias[n] : 0.f);
-                            v[u] = GELU ? gelu_erf_u(x) : x;
-                        }
-                        const int phys = j4 ^ ((lane >> 1) & 3);
-                        *reinterpret_cast<float4*>(stg + lane * 16 + phys * 4) = make_float4(v[0], v[1], v[2], v[3]);
+                    for (int j = 0; j < 16; ++j) {
+                        const float x = v[j] * w_unscale + __shfl_sync(0xffffffffu, pass < 2 ? b_lo : b_hi, (pass * 16 + j) & 31);
+                        v[j] = GELU ? gelu_erf_u(x) : x;
                     }
-                    __syncwarp();
+                }
+                if (lane == 0) bulk_wait_read_all();          // the previous box has left the slot
+                __syncwarp();
+                if (split_out && !raw) {
+                    // h1 at stg, h2 at stg + 1024: 32 B rows; SWIZZLE_32B puts 16-byte chunk c of row r at c ^ ((r >> 2) & 1)
+                    uint32_t p1[8], p2[8];
 #pragma unroll
-                    for (int i = 0; i < 4; ++i) {
-                        const int rr = i * 8 + (lane >> 2), chk = lane & 3;
-                        const float4 o = *reinterpret_cast<const float4*>(stg + rr * 16 + (chk ^ ((rr >> 1) & 3)) * 4);
-                        const int row = row0 + rr;
-                        const int n = nb + pass * 16 + chk * 4;
-                        if (row < M && n < N) {
-                            const int64_t off = (int64_t)row * ldc + n;
-                            if (n + 3 < N) {
-                                if (C) *reinterpret_cast<float4*>(C + off) = o;
-                                if (C_h1) {
-                                    __half h1[4], h2[4];
-                                    int ov = 0;
-                                    split_half(o.x, h1[0], h2[0], &ov); split_half(o.y, h1[1], h2[1], &ov);
-                                    split_half(o.z, h1[2], h2[2], &ov); split_half(o.w, h1[3], h2[3], &ov);
-                                    if (ov) atomicExch(overflow, 1);
-                                    *reinterpret_cast<uint2*>(C_h1 + off) = make_uint2(
-                                        (uint32_t)__half_as_ushort(h1[0]) | ((uint32_t)__half_as_ushort(h1[1]) << 16),
-                                        (uint32_t)__half_as_ushort(h1[2]) | ((uint32_t)__half_as_ushort(h1[3]) << 16));
-                                    *reinterpret_cast<uint2*>(C_h2 + off) = make_uint2(
-                                        (uint32_t)__half_as_ushort(h2[0]) | ((uint32_t)__half_as_ushort(h2[1]) << 16),
-                                        (uint32_t)__half_as_ushort(h2[2]) | ((uint32_t)__half_as_ushort(h2[3]) << 16));
-                                }
-                            } else {
-                                const float vv[4] = {o.x, o.y, o.z, o.w};
-                                for (int u = 0; u < 4; ++u) if (n + u < N) {
-                                    if (C) C[off + u] = vv[u];
-                                    if (C_h1) { __half a, bh; int ov = 0; split_half(vv[u], a, bh, &ov); if (ov) atomicExch(overflow, 1); C_h1[off + u] = a; C_h2[off + u] = bh; }
-                                }
-                            }
-                        }
+                    for (int j = 0; j < 16; j += 2) {
+                        __half a1, a2, c1, c2;
+                        split_half(v[j], a1, a2, &ov);
+                        split_half(v[j + 1], c1, c2, &ov);
+                        p1[j / 2] = pack_half2(a1, c1);
+                        p2[j / 2] = pack_half2(a2, c2);
                     }
-                    __syncwarp();
+#pragma unroll
+                    for (int c = 0; c < 2; ++c) {
+                        const uint32_t off = (uint32_t)(lane * 32 + ((c ^ ((lane >> 2) & 1)) * 16));
+                        st_shared_v4(stg + off, p1[4 * c], p1[4 * c + 1], p1[4 * c + 2], p1[4 * c + 3]);
+                        st_shared_v4(stg + 1024 + off, p2[4 * c], p2[4 * c + 1], p2[4 * c + 2], p2[4 * c + 3]);
+                    }
+                } else {
+                    // fp32: 64 B rows; SWIZZLE_64B puts 16-byte chunk c of row r at c ^ ((r >> 1) & 3)
+#pragma unroll
+                    for (int c = 0; c < 4; ++c)
+                        st_shared_v4(stg + (uint32_t)(lane * 64 + ((c ^ ((lane >> 1) & 3)) * 16)), __float_as_uint(v[4 * c]),
+                                     __float_as_uint(v[4 * c + 1]), __float_as_uint(v[4 * c + 2]), __float_as_uint(v[4 * c + 3]));
+                }
+                fence_proxy_async_smem();
+                __syncwarp();
+                if (lane == 0) {
+                    if (raw) tma_store_2d(&tmPart, stg, col, row0);
+                    else if (split_out) { tma_store_2d(&tmOut, stg, col, row0); tma_store_2d(&tmOut2, stg + 1024, col, row0); }
+                    else tma_store_2d(&tmOut, stg, col, row0);
+                    bulk_commit();
                 }
             }
+            if (__any_sync(0xffffffffu, ov) && lane == 0) atomicExch(overflow, 1);
         }
+        if (lane == 0) bulk_wait_all();
     }
     tc_fence_before();
     __syncthreads();
